@@ -19,6 +19,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True    # the benchmark writes nothing into the tree it runs from (it may be read-only)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 import torch                      # noqa: E402
@@ -50,12 +51,20 @@ def parse():
     ap.add_argument("--envmap_w", type=int, default=None)
     ap.add_argument("--no-strong", dest="no_strong", action="store_true",
                     help="N > 1: skip the additional strong-scaling measurement")
+    ap.add_argument("--reference", default=None, metavar="DIR",
+                    help="a checkout of the original TensoIR project: adds the PyTorch-on-GPU denominator (its unmodified "
+                         "modules on the same GPU, field and batches)")
     ap.add_argument("--no-torch-reference", dest="no_torch_reference", action="store_true",
-                    help="skip the PyTorch-on-GPU denominator (unmodified reference from baseline/_ref)")
+                    help="skip the PyTorch-on-GPU denominator even with --reference")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", default=None, metavar="DIR",
+                    help="write what the timed path computed in its last step to DIR/<name>.npy (float32; the parameters "
+                         "after the step as a fixed seeded sample), so that two builds can be compared output for output")
     ap.add_argument("--scaling", choices=["weak", "strong"], default="weak",
                     help="weak: every rank renders its own --batch rays (global batch = batch x N); strong: the --batch "
                          "rays of a step are split over the ranks (SURVEY.md 8e: same draw on all ranks, contiguous slices)")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     if a.envmap_h is None:
         a.envmap_h, a.envmap_w = (8, 16) if a.config == 3 else (16, 32)
     return a
@@ -332,6 +341,11 @@ def measure(a, model, n_lights, rank, world, local, dev, scaling, with_e2e, cloc
     target = torch.full((per_rank, 3), 0.5, device=dev)
     counters = ops.new_counters(dev)
     model.__dict__["_tir_counters"] = counters
+    last = {}          # the renderer's outputs and the loss of the most recent step
+
+    def loss_fn(ret, m):
+        last["ret"] = ret
+        return loss_of(ret, target, m, l1_in_optimizer=fused_opt)
     # production mode of the marches: work that would only feed the mask / density COUNTERS is skipped (the rest of a ray
     # whose transmittance is exactly 0); rays, appearance samples and every output are unaffected.
     model.__dict__["_tir_lean"] = True
@@ -340,9 +354,8 @@ def measure(a, model, n_lights, rank, world, local, dev, scaling, with_e2e, cloc
     if not a.eager:
         # whole-step CUDA graph: static-capacity sample lists, host randoms staged into device buffers, replay
         from tensoir_b200.static_step import StaticTrainStep
-        graphed = StaticTrainStep(model, opt, per_rank, n_s, Args,
-                                  lambda ret, m: loss_of(ret, target, m, l1_in_optimizer=fused_opt),
-                                  grad_bucket=bucket, device=dev)
+        # a replay rewrites the tensors the captured loss_fn saw: last["ret"] then holds the latest replay's outputs
+        graphed = StaticTrainStep(model, opt, per_rank, n_s, Args, loss_fn, grad_bucket=bucket, device=dev)
         # lists sized from 8 batches x 1.5; they grow by themselves (high-water marks, re-capture) and a replay whose
         # lists did not fit is an exact no-op that is redone (static_step.py) - never a silently different step
         graphed.calibrate(host_batches[:8])
@@ -350,16 +363,18 @@ def measure(a, model, n_lights, rank, world, local, dev, scaling, with_e2e, cloc
 
     def step(rays, li):
         if graphed is not None:
-            return graphed.run(rays, li)
+            last["loss"] = graphed.run(rays, li)
+            return last["loss"]
         ret = Renderer_TensoIR_train(rays, None, li, model, N_samples=n_s, white_bg=True, is_train=True,
                                      is_relight=True, sample_method='stratified_sampling', chunk_size=160000,
                                      device=dev, args=Args)
-        loss = loss_of(ret, target, model, l1_in_optimizer=fused_opt)
+        loss = loss_fn(ret, model)
         opt.zero_grad(set_to_none=False)
         loss.backward()
         if bucket is not None:
             bucket.all_reduce_mean()
         opt.step()
+        last["loss"] = loss
         return loss
 
     def barrier():
@@ -411,6 +426,9 @@ def measure(a, model, n_lights, rank, world, local, dev, scaling, with_e2e, cloc
     out = {"scaling": scaling, "ms": ms, "cnt": cnt, "launches": launches, "per_rank": per_rank,
            "value": cnt["rays"] / (ms * 1e-3),   # TIR_CNT_RAYS counts every marched ray: primary + secondary
            "last_batch": dev_batches[-1], "n_s": n_s}
+    if a.dump_outputs is not None and rank == 0:
+        # before the end-to-end arm trains the model further
+        out["outputs"] = train_step_outputs(last["ret"], last["loss"], model)
     if with_e2e:
         # ---- end-to-end arm: pinned HOST buffers through the public boundary, loss read back every step.
         # Default: the host sends (view, pixel, light) ids - 12 B/ray - and the rays are generated on the device
@@ -465,10 +483,10 @@ def measure(a, model, n_lights, rank, world, local, dev, scaling, with_e2e, cloc
 
 
 def torch_gpu_reference(a, model, n_lights):
-    """The unmodified reference (baseline/_ref) on the same GPU / field / batches, in a subprocess (its `models` and
-    `renderer` modules must not meet tensoir_b200's).  None when the reference copy did not travel to this box."""
-    ref = os.path.join(ROOT, "baseline", "_ref")
-    if not os.path.isdir(ref) or a.config not in (2, 3) or (a.envmap_h, a.envmap_w) != (16, 32):
+    """The unmodified reference (the checkout given by --reference) on the same GPU / field / batches, in a subprocess
+    (its `models` and `renderer` modules must not meet tensoir_b200's).  None without --reference."""
+    ref = a.reference and os.path.abspath(a.reference)
+    if not ref or a.config not in (2, 3) or (a.envmap_h, a.envmap_w) != (16, 32):
         return None          # (the reference's checkpoint kwargs carry no envmap size: only its 16x32 default is comparable)
     import tempfile
     tmp = tempfile.mkdtemp(prefix="tir_ref_")
@@ -569,12 +587,40 @@ def main():
         if "ms_per_step" in ref_gpu:
             ref_gpu["speedup_ms_per_step"] = ref_gpu["ms_per_step"] / (ms / a.steps)
         line["torch_gpu_reference"] = ref_gpu
+    if a.dump_outputs is not None:
+        write_outputs(a.dump_outputs, m["outputs"])
     if not a.no_cpu_baseline and world == 1:
         cb = cpu_baseline(a, steps=2, warmup=1)
         line["cpu_baseline"] = {"value": cb["value"], "unit": UNIT, "cores": cb["cores"], "kind": "port",
                                 "sample": cb["sample"]}
     print(json.dumps(line))
     finish()
+
+
+def train_step_outputs(ret, loss, model, n_sample=1 << 16, seed=0):
+    """What a caller of the training step receives from its last call, as float32 arrays: the loss, every tensor the
+    renderer returned, and each parameter after the optimiser step - all of a small one, a fixed seeded sample of
+    ``n_sample`` entries (the same positions in every run) of a larger one."""
+    out = {"loss": loss}
+    out.update((k, v) for k, v in ret.items() if torch.is_tensor(v))
+    g = torch.Generator().manual_seed(seed)
+    for k, p in model.named_parameters():
+        flat = p.detach().reshape(-1)
+        if flat.numel() > n_sample:
+            flat = flat[torch.randperm(flat.numel(), generator=g)[:n_sample].sort().values.to(flat.device)]
+        out["param." + k] = flat
+    return {k: v.detach().float().cpu().numpy() for k, v in out.items()}
+
+
+def write_outputs(path, arrays, limit=64 << 20):
+    """DIR/<name>.npy for every array; refuses to write more than ``limit`` bytes in all."""
+    import numpy as np
+    total = sum(v.nbytes for v in arrays.values())
+    if total > limit:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs exceed the {limit}-byte limit")
+    os.makedirs(path, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), np.ascontiguousarray(v))
 
 
 def synthetic_hdr(h=1024, w=2048, seed=20211202):
@@ -636,7 +682,7 @@ def run_relight_pass(a, rank, world, local, dev):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for c in batches:
-            step(c, read_back)
+            last["img"] = step(c, read_back)
         e1.record()
         torch.cuda.synchronize()
         if world > 1:
@@ -648,6 +694,7 @@ def run_relight_pass(a, rank, world, local, dev):
             dist.all_reduce(c, op=dist.ReduceOp.SUM)
         return float(t.item()), ops.counters_dict(c)
 
+    last = {}
     dev_chunks = [c.to(dev) for c in chunks[:total]]
     clocks = ClockSampler(local) if rank == 0 else None
     if clocks is not None:
@@ -657,6 +704,8 @@ def run_relight_pass(a, rank, world, local, dev):
     if clocks is not None:
         clocks.mark()
     ms, cnt = timed(dev_chunks[a.warmup:], False)
+    if a.dump_outputs is not None and rank == 0:
+        write_outputs(a.dump_outputs, {"relit_rgb": last["img"].float().cpu().numpy()})
     for c in pinned[:a.warmup]:
         step(c, True)
     ms_e2e, cnt_e2e = timed(pinned[a.warmup:total], True)

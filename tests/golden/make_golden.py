@@ -1,14 +1,18 @@
-"""Generate golden fixtures by running the REAL reference (imported from /root/reference).
+"""Generate golden fixtures by running the REAL reference (a checkout of the original TensoIR project):
 
-Run in the build container only (the GPU box has no /root/reference):
-
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <path of the original project> [<output directory>]
 
 Writes tests/golden/*.pt: small seeded inputs, the reference model's state_dict / alpha mask,
 and the reference's outputs for every hot-path function (SURVEY.md §8a).  The oracle
 (oracle/tensoir_oracle.py) is replayed against these in tests/test_oracle_golden.py, and the
-CUDA path is checked against the same fixtures in the -m gpu tests.
+CUDA path is checked against the same fixtures in the -m gpu tests.  Also writes the names the
+reference's own modules import from ``models.*`` (reference_imports.json) and the reference's
+grid_sample outside [-1, 1] (grid_sample_outside.pt), which tests/test_dropin_cpu.py checks
+dropin/ against.  No file may exceed 1 MB: the rotated model's state_dict is stored in a file of
+its own, and its training gradients as a fixed sample (see ``sample_grads``).
 """
+import ast
+import json
 import os
 import sys
 import types
@@ -18,12 +22,13 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 REPO = os.path.dirname(os.path.dirname(HERE))
-REF = "/root/reference"
+REF = None          # the original project's checkout, set by main()
 sys.path.insert(0, REPO)
+GRAD_SAMPLE = 2048  # gradient entries kept per tensor with more entries than this: the largest half + a seeded rest
 
 
 def import_reference():
-    """Put /root/reference on sys.path with the stubs SURVEY.md §8c lists."""
+    """Put the reference on sys.path with the stubs SURVEY.md §8c lists."""
     kornia = types.ModuleType("kornia")
 
     def create_meshgrid(h, w, normalized_coordinates=True, device=None, dtype=torch.float32):
@@ -85,11 +90,70 @@ def rays_for(n, seed=3):
     return torch.cat(out, 0)
 
 
+def sample_grads(grads, n=GRAD_SAMPLE, seed=5):
+    """name -> None or {idx, val, absmax}: every entry of a small gradient; of a larger one the n // 2 entries of
+    largest magnitude plus n - n // 2 seeded uniform draws from the rest.  ``absmax`` is the whole tensor's, so a
+    relative error keeps the scale of the full comparison."""
+    g = torch.Generator().manual_seed(seed)
+    out = {}
+    for k, w in grads.items():
+        if w is None:
+            out[k] = None
+            continue
+        flat = w.reshape(-1)
+        if flat.numel() <= n:
+            idx = torch.arange(flat.numel())
+        else:
+            top = flat.abs().topk(n // 2).indices
+            rest = torch.ones(flat.numel(), dtype=torch.bool)
+            rest[top] = False
+            rest = rest.nonzero().reshape(-1)
+            idx = torch.cat([top, rest[torch.randperm(rest.numel(), generator=g)[:n - n // 2]]]).sort().values
+        out[k] = dict(idx=idx.to(torch.int32), val=flat[idx].clone(), absmax=flat.abs().max().clone())
+    return out
+
+
+def reference_imports():
+    """{importer: [[module, [names]]]}: every ``from models.X import a, b`` in the reference outside models/ (the
+    modules an unchanged script loads through dropin/).  Star imports name nothing and are left out."""
+    out = {}
+    for d, _, files in sorted(os.walk(REF)):
+        rel = os.path.relpath(d, REF)
+        top = rel.split(os.sep)[0]
+        if top in ("models", "__pycache__") or (top != "." and top.startswith(".")):
+            continue
+        for fn in sorted(files):
+            if not fn.endswith(".py"):
+                continue
+            path = os.path.join(d, fn)
+            for node in ast.walk(ast.parse(open(path).read(), path)):
+                if isinstance(node, ast.ImportFrom) and (node.module or "").startswith("models."):
+                    names = [a.name for a in node.names if a.name != "*"]
+                    if names:
+                        out.setdefault(os.path.relpath(path, REF), []).append([node.module, names])
+    return out
+
+
+def grid_sample_outside(ru):
+    """The reference's clamped grid_sample (models/relight_utils.py) on coordinates inside and outside [-1, 1]."""
+    g = torch.Generator().manual_seed(0)
+    img = torch.randn(2, 5, 7, 9, generator=g)
+    grid = torch.rand(2, 6, 4, 2, generator=g) * 3 - 1.5
+    return dict(img=img, grid=grid, out=ru.grid_sample(img, grid).detach().clone())
+
+
 def tolist(t):
     return [x.detach().clone() if torch.is_tensor(x) else x for x in t]
 
 
 def main():
+    global REF, HERE
+    if len(sys.argv) < 2:
+        raise SystemExit(__doc__)
+    REF = os.path.abspath(sys.argv[1])
+    if len(sys.argv) > 2:
+        HERE = os.path.abspath(sys.argv[2])
+        os.makedirs(HERE, exist_ok=True)
     ru, rot, gen, ini = import_reference()
     import renderer as ref_renderer
     out = {}
@@ -268,6 +332,9 @@ def main():
                           density_plane1=m2.density_plane[1].detach().clone(),
                           app_line0=m2.app_line[0].detach().clone())
     out["rotated"] = fx
+    torch.save(fx.pop("state_dict"), os.path.join(HERE, "rotated_g24_state.pt"))
+    fx["state_dict"] = "rotated_g24_state.pt"          # resolved by tests/gpu_helpers.load_fixture
+    fx["renderer_train_grads_sample"] = sample_grads(fx.pop("renderer_train_grads"))
     torch.save(fx, os.path.join(HERE, "rotated_g24.pt"))
 
     # ---------------- general multi-light model (boundary smoke) -------------------------
@@ -312,7 +379,11 @@ def main():
               forward_nomask=(rgb0.detach().clone(), dep0.detach().clone()),
               forward_mask=(rgb1.detach().clone(), dep1.detach().clone()))
     torch.save(fi, os.path.join(HERE, "init_g24.pt"))
-    for n in ("rotated_g24.pt", "general_g20.pt", "init_g24.pt"):
+    torch.save(grid_sample_outside(ru), os.path.join(HERE, "grid_sample_outside.pt"))
+    with open(os.path.join(HERE, "reference_imports.json"), "w") as fh:
+        json.dump(reference_imports(), fh, indent=1, sort_keys=True)
+        fh.write("\n")
+    for n in ("rotated_g24.pt", "rotated_g24_state.pt", "general_g20.pt", "init_g24.pt", "grid_sample_outside.pt"):
         print(n, os.path.getsize(os.path.join(HERE, n)) // 1024, "KiB")
 
 

@@ -208,13 +208,14 @@ def test_boundary_train_step_grads(golden_rotated):
     close(loss, fx["renderer_train_loss"], TOL, "loss")
     n, worst = 0, {}
     for k, p in m.named_parameters():
-        w = fx["renderer_train_grads"][k]
+        w = fx["renderer_train_grads_sample"][k]
         if w is None:
             assert p.grad is None or float(p.grad.abs().max()) == 0.0, k
             continue
-        g = p.grad.detach().cpu()
-        scale = float(w.abs().max()) + 1e-12
-        err = float((g - w).abs().max()) / scale
+        g = p.grad.detach().cpu().reshape(-1)
+        scale = float(w["absmax"]) + 1e-12
+        err = max(float((g[w["idx"].long()] - w["val"]).abs().max()), abs(float(g.abs().max()) - float(w["absmax"])))
+        err /= scale
         worst[k] = err
         n += 1
     assert n >= 20

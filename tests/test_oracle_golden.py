@@ -109,11 +109,12 @@ def test_boundary_train_with_grads(golden_rotated):
     eq(loss.detach(), fx["renderer_train_loss"])
     params = named_oracle_params(f)
     n_checked = 0
-    for k, g in fx["renderer_train_grads"].items():
+    for k, g in fx["renderer_train_grads_sample"].items():
         if g is None:
             assert params[k].grad is None or float(params[k].grad.abs().max()) == 0.0
             continue
-        eq(params[k].grad, g, tol=1e-6)
+        eq(params[k].grad.reshape(-1)[g["idx"].long()], g["val"], tol=1e-6)
+        eq(params[k].grad.abs().max(), g["absmax"], tol=1e-6)
         n_checked += 1
     assert n_checked >= 20
 

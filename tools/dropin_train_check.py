@@ -1,4 +1,4 @@
-"""Drop-in check on the GPU box: the UNMODIFIED reference script `train_tensoIR.py` (copy under baseline/_ref) is run
+"""Drop-in check on a GPU: the UNMODIFIED reference script `train_tensoIR.py` (of the checkout given by --reference) is run
 twice for a few iterations on a small synthetic on-disk dataset in the reference's own format —
   A. with `dropin/` first on PYTHONPATH: `models.*` / `renderer` resolve to tensoir_b200 (CUDA kernels),
   B. against the reference's own modules (eager PyTorch on the same GPU) —
@@ -6,7 +6,7 @@ same seeds, same config, and the per-iteration training losses written by the sc
 The run crosses the script's `update_AlphaMask_list[0]` iteration, so both phases (radiance-only, then relight with
 secondary rays), `filtering_rays`, `updateAlphaMask`, `shrink` and `save` are exercised through the drop-in surface.
 
-    python tools/dropin_train_check.py [--iters 24] [--out profiles/r2_dropin_train_check.json]
+    python tools/dropin_train_check.py --reference <original project> [--iters 24] [--out profiles/r2_dropin_train_check.json]
 """
 import argparse
 import json
@@ -19,7 +19,7 @@ import tempfile
 import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(ROOT, "baseline", "_ref")
+REF = None           # the original project's checkout (--reference)
 STUBS = os.path.join(ROOT, "tools", "ref_stubs")
 
 
@@ -133,14 +133,16 @@ def run(arm, cfg, env_paths, log):
 
 
 def main():
+    global REF
     ap = argparse.ArgumentParser()
+    ap.add_argument("--reference", required=True, help="a checkout of the original TensoIR project")
     ap.add_argument("--iters", type=int, default=24)
     ap.add_argument("--out", default=None)
     ap.add_argument("--keep", action="store_true")
     a = ap.parse_args()
-    if not os.path.isdir(REF):
-        print(json.dumps({"unavailable": "baseline/_ref (copy of the reference tree) is not present"}))
-        return 0
+    REF = os.path.abspath(a.reference)
+    if not os.path.isfile(os.path.join(REF, "train_tensoIR.py")):
+        raise SystemExit(f"{REF}: not a checkout of the original project (no train_tensoIR.py)")
     tmp = tempfile.mkdtemp(prefix="tir_dropin_")
     scan, hdr = make_dataset(tmp)
     ckpt = os.path.join(tmp, "start.th")

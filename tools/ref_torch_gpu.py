@@ -1,7 +1,8 @@
-"""PyTorch-on-B200 denominator: the UNMODIFIED reference modules (baseline/_ref: models.tensoRF_rotated_lights +
+"""PyTorch-on-B200 denominator: the UNMODIFIED reference modules (bench.py --reference: models.tensoRF_rotated_lights +
 renderer.Renderer_TensoIR_train, eager PyTorch, no tensoir_b200 code on the path) timed on the same GPU, the same
 field (loaded from a checkpoint bench.py wrote in the reference's format) and the same ray batches as bench.py.
-Run by bench.py in a subprocess:  PYTHONPATH=tools/ref_stubs:baseline/_ref:<repo>  python -P tools/ref_torch_gpu.py ..."""
+Run by bench.py in a subprocess, from the reference's directory:
+    PYTHONPATH=tools/ref_stubs:<reference>:<repo>  python -P tools/ref_torch_gpu.py ..."""
 import argparse
 import json
 import os
@@ -22,7 +23,7 @@ a = ap.parse_args()
 from models.tensoRF_rotated_lights import TensorVMSplit, AlphaGridMask   # noqa: E402,F401  (the reference's own)
 from renderer import Renderer_TensoIR_train                               # noqa: E402
 import models.tensoRF_rotated_lights as _m                                # noqa: E402
-assert "baseline" in os.path.abspath(_m.__file__), _m.__file__
+assert os.path.abspath(_m.__file__).startswith(os.getcwd() + os.sep), _m.__file__     # not dropin/'s
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.append(ROOT)
@@ -62,6 +63,6 @@ for it in range(a.warmup + a.steps):
     torch.cuda.synchronize()
     if it >= a.warmup:
         ts.append(time.perf_counter() - t0)
-print(json.dumps({"impl": "unmodified reference modules (baseline/_ref), eager PyTorch, same B200 / field / batches",
+print(json.dumps({"impl": "unmodified reference modules, eager PyTorch, same B200 / field / batches",
                   "ms_per_step": 1e3 * sum(ts) / len(ts), "steps": a.steps, "warmup": a.warmup, "loss": float(loss),
                   "peak_mem_GB": torch.cuda.max_memory_allocated() / 1e9}))
